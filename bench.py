@@ -8,7 +8,7 @@ One STEP = one pass of the hot path over one synthetic batch per GPU:
   + backward through MTA and the student stack (all BiFPN parameter gradients + dL/dC3..C5)
   + (N > 1) one NCCL all-reduce of the flat student gradient buffer.
 
-    python bench.py [--gpus N --steps K --warmup W] [--dtype f32|bf16] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--dtype f32|bf16] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU port of the reference algorithm (oracle/) on the
@@ -257,10 +257,33 @@ def bind_to_gpu_numa_node(gpu_index):
         return "not bound (%s: %s)" % (type(e).__name__, str(e)[:80])
 
 
-def measure(B, args, rank, world, dev, dtype, min_timed_s):
+DUMP_SAMPLE = 1 << 20   # elements kept of each input gradient (dL/dC3 alone is 57 MB in fp32 at batch 32)
+
+
+def dump_outputs(out_dir, kd, step, student, xs):
+    """Write what the last timed step handed its caller as out_dir/<name>.npy (float32): the [teacher, level] MTA losses it
+    returned, the averaged flat student gradient, dL/dC3..C5 (a fixed, seeded sample of each, in NCHW element order), and
+    the student's parameters and BatchNorm running statistics as that step left them.  Gradients and parameters differ
+    in the last bits from run to run (atomic accumulation in the backward): compare dumps within a tolerance."""
+    import numpy as np
+    arrays = {"kd_losses": kd, "student_grad": step.flat_grad,
+              "student_params": torch.cat([p.detach().flatten() for p in student.parameters()]),
+              "student_bn_stats": torch.cat([b.flatten() for b in student.buffers() if b.is_floating_point()])}
+    gen = torch.Generator().manual_seed(0)
+    for name, x in zip(("c3", "c4", "c5"), xs):
+        g = x.grad.flatten()
+        idx = torch.randperm(g.numel(), generator=gen)[:DUMP_SAMPLE].sort().values
+        arrays["input_grad_" + name] = g[idx.to(g.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
+def measure(B, args, rank, world, dev, dtype, min_timed_s, dump_dir=None):
     """Everything measured at one per-GPU batch size: resident (device-timed) step, end-to-end step, per-kernel
     instrumented pass.  Timed regions are blocks of EXACTLY args.steps steps bracketed by barrier + synchronize; blocks are
-    repeated until >= min_timed_s seconds have been timed and the MEDIAN block is reported (max over ranks per block)."""
+    repeated until >= min_timed_s seconds have been timed and the MEDIAN block is reported (max over ranks per block).
+    With `dump_dir`, rank 0 writes the outputs of the last resident step there (dump_outputs)."""
     import mm_distillnet_b200 as mmd
     from mm_distillnet_b200 import _lib
     esize = 4 if dtype == torch.float32 else 2
@@ -340,10 +363,10 @@ def measure(B, args, rank, world, dev, dtype, min_timed_s):
         # into the set that is not running (no staging-to-static copy); the resident leg replays one of them
         step.capture(dev_s, dev_t, warmup=max(args.warmup, 3), double_buffer=not args.no_prefetch)
 
+    last_kd = [None]
+
     def resident_step():
-        if use_graph:
-            return step.replay()
-        return eager_step()
+        last_kd[0] = step.replay() if use_graph else eager_step()
 
     host_loss = torch.empty(N_TEACHERS, 5, dtype=torch.float32).pin_memory()
     e2e_i, e2e_total = [0], [0]
@@ -374,6 +397,8 @@ def measure(B, args, rank, world, dev, dtype, min_timed_s):
     ms, blocks = timed(resident_step, args.steps)
     clocks = sampler.stop() if sampler else None
     torch.cuda.synchronize()
+    if dump_dir is not None and rank == 0:   # before the legs below run more steps on the same student
+        dump_outputs(dump_dir, last_kd[0], step, student, step.graph_inputs() if use_graph else dev_s)
     l0 = mmd.launch_count()   # replayed launches never pass through the library's host-side counter: count one eager step
     eager_step()
     torch.cuda.synchronize()
@@ -475,7 +500,7 @@ def run_ours(args, rank, world, local_rank):
     dtype = torch.float32 if args.dtype == "f32" else torch.bfloat16
     B = args.batch
     numa = bind_to_gpu_numa_node(local_rank) if world > 1 else "single rank: not bound"
-    main_r = measure(B, args, rank, world, dev, dtype, args.min_seconds)
+    main_r = measure(B, args, rank, world, dev, dtype, args.min_seconds, args.dump_outputs)
     cfg2 = None
     if B != 16 and not args.no_cfg2:   # BASELINE configs[1]: the microbench batch, same run, shorter timed region
         cfg2 = measure(16, args, rank, world, dev, dtype, min(args.min_seconds, 1.0))
@@ -537,7 +562,9 @@ def run_ours(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=300, help="timed steps: every timed leg runs exactly this many; the "
+                    "default times about 2 s of the batch-32 step (6.6 ms per step on a B200 at a 1000 W power limit), a "
+                    "window of a fraction of a second measures clock and scheduler noise as much as the step")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--dtype", default="bf16", choices=["f32", "bf16"],
@@ -545,8 +572,11 @@ def main():
                          "bf16 is the tensor-core product path (BASELINE cfg 3), f32 the bit-level parity mode")
     ap.add_argument("--batch", type=int, default=32, help="samples per GPU per step (cfg3/cfg4: 32; cfg2's 16 is measured "
                     "in the same run and reported as cfg2_b16)")
-    ap.add_argument("--min-seconds", type=float, default=2.0, help="repeat the timed block of K steps until this many "
-                    "seconds have been timed; the median block is reported")
+    ap.add_argument("--min-seconds", type=float, default=0.0, help="repeat the timed block of K steps until this many "
+                    "seconds have been timed; the median block is reported (default: one block, exactly K timed steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                    "(float32, see dump_outputs) to compare builds on identical inputs, within a tolerance: the backward "
+                    "accumulates with atomics, so gradients and updated parameters vary in the last bits from run to run")
     ap.add_argument("--no-cfg2", action="store_true", help="skip the extra cfg2 (batch 16) measurement")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-optimizer", action="store_true", help="end the step at the averaged gradients (no Adam update)")
@@ -559,6 +589,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA step (--impl ours)")
         run_reference(args, rank)
         return
     if world > 1:

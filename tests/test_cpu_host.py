@@ -307,10 +307,71 @@ def test_library_staleness_is_a_content_hash():
     assert not _lib.is_stale() and saved.strip() == _lib.source_hash()
 
 
-REF = "/root/reference"
+def _reference_d2_state():
+    """(parameters, buffers) of the reference D2 model's bifpn / regressor / classifier as recorded from the reference
+    modules in the golden fixtures (oracle/make_golden.py loads each module strictly, then stores every parameter's
+    gradient in named_parameters order and every BatchNorm buffer): [(key, array)], parameter arrays shaped like the
+    parameters.  stack2_c112 holds a first cell ("0.") and a later one ("1."), reg_c112 / cls_c112 the D2 heads (112
+    channels, 9 anchors, 3 layers, 20 classes)."""
+    fixtures = {n: H.golden(n) for n in ("stack2_c112", "reg_c112", "cls_c112")}
+    parts = [("bifpn.%d." % i, "stack2_c112", "0." if i == 0 else "1.") for i in range(5)] + \
+        [("regressor.", "reg_c112", ""), ("classifier.", "cls_c112", "")]
+    params, bufs = [], []
+    for prefix, fixture, src in parts:
+        for k, v in fixtures[fixture].items():
+            for tag, out in (("pgrad_" + src, params), ("buf_" + src, bufs)):
+                if k.startswith(tag):
+                    out.append((prefix + k[len(tag):], v))
+    return params, bufs
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="the reference tree exists in the build container only")
+def test_d2_model_matches_the_reference_state_dict():
+    """patch_reference(heads=True) on a stand-in YetAnotherEfficientDet that builds the BiFPN and the heads as the
+    reference's constructor does (src/YetAnotherEfficientDet.py:611-629 sizes, :639-652 modules): the D2 model has the
+    reference's parameter names in the reference's order, its shapes and its buffers (golden fixtures), loads a state_dict
+    with exactly those keys strictly, and other compound coefficients / too wide headers fail at construction."""
+    import types
+    det = types.ModuleType("det")
+
+    class YetAnotherEfficientDet(torch.nn.Module):
+        def __init__(self, num_classes=20, compound_coef=2):
+            super().__init__()
+            C = [64, 88, 112][compound_coef]
+            cc = [[40, 112, 320], [40, 112, 320], [48, 120, 352]][compound_coef]
+            self.bifpn = torch.nn.Sequential(*[det.BiFPN(C, cc, True if i == 0 else False) for i in range([3, 4, 5][compound_coef])])
+            self.regressor = det.Regressor(in_channels=C, num_anchors=9, num_layers=3)
+            self.classifier = det.Classifier(in_channels=C, num_anchors=9, num_classes=num_classes, num_layers=3)
+
+    det.YetAnotherEfficientDet = YetAnotherEfficientDet
+    det.BiFPN = det.Regressor = det.Classifier = object
+    loss = types.ModuleType("loss")
+    loss.MTALoss = object
+    mmd.patch_reference(det, loss, types.ModuleType("utils"), heads=True)
+    params, bufs = _reference_d2_state()
+    assert len(params) == 72 + 4 * 48 + 2 * 42 and len(bufs) == 42 + 4 * 24 + 2 * 45
+    m = det.YetAnotherEfficientDet(num_classes=20, compound_coef=2)
+    assert isinstance(m.bifpn, mmd.BiFPNStack) and len(m.bifpn) == 5
+    assert isinstance(m.regressor, mmd.Regressor) and isinstance(m.classifier, mmd.Classifier)
+    assert [(k, tuple(p.shape)) for k, p in m.named_parameters()] == [(k, v.shape) for k, v in params]
+    sd = m.state_dict()
+    pkeys = {k for k, _ in params}
+    assert {(k, tuple(v.shape)) for k, v in sd.items() if k not in pkeys} == {(k, v.shape) for k, v in bufs}
+    ref_sd = {k: torch.from_numpy(v) for k, v in params + bufs}
+    assert set(sd) == set(ref_sd)
+    m.load_state_dict(ref_sd, strict=True)
+    assert all(torch.equal(v, ref_sd[k]) for k, v in m.state_dict().items())
+    with pytest.raises(NotImplementedError):   # D0: 64 channels
+        det.YetAnotherEfficientDet(num_classes=20, compound_coef=0)
+    with pytest.raises(NotImplementedError):   # 9 x 90 = 810 header channels: more than two C-row halves
+        det.YetAnotherEfficientDet(num_classes=90, compound_coef=2)
+
+
+# a checkout of the reference (robot-learning-freiburg/MM-DistillNet) and its Python dependencies; not part of this repository
+REF = os.environ.get("MMD_REFERENCE_SRC", "")
+
+
+@pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "src"))),
+                    reason="set MMD_REFERENCE_SRC to a checkout of the reference MM-DistillNet to run this test")
 def test_patch_reference_on_the_real_modules():
     """patch_reference() on the REAL src.* modules (not fakes): the patched YetAnotherEfficientDet(D2) has the same
     state_dict keys / shapes as the unpatched one, loads its state_dict strictly, holds a fused BiFPNStack, refuses CPU
