@@ -86,8 +86,13 @@ def param_class(k):
         "proj" if ".0.conv" in k else "bn"
 
 
+def input_tile(x):
+    """(TW, TH) of the tiles the backward uses at x's level: the whole sample on a run-time-geometry level."""
+    return H.pick_geom(x.shape[2], x.shape[3]) or (x.shape[3], x.shape[2])
+
+
 def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channels_last=False, ref64=True,
-                      fw_mode="ones", force_argmax=None, attention=True):
+                      fw_mode="ones", force_argmax=None, attention=True, ref32=True, tile_metrics=False, teachers=0):
     """CUDA stack vs the oracle (fp64 and fp32) on D2-shaped random data.  Returns metrics for ours and, for
     calibration, for the fp32 oracle against the fp64 oracle.
     force_argmax (default on): every oracle run takes its max-pool arg-max from the window indices the CUDA forward itself
@@ -95,36 +100,57 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
     differently by two summation orders (fp32: 1e-4 .. 1e-3 jumps of every gradient; bf16 storage: the dominant part of
     the gradient error) no longer hides the arithmetic error of the kernels.  The forward comparison of the train
     outputs uses the hinted oracle too: its values differ from the true maxima by the top-2 gap of the flipped windows
-    only (~1e-7 fp32); the eval forward is always compared against the plain, unhinted oracle."""
+    only (~1e-7 fp32); the eval forward is always compared against the plain, unhinted oracle.
+    s3: the P3 side, or (H3, W3) for a non-square pyramid (level i is (H3 >> i) x (W3 >> i)).
+    ref32=False skips the fp32 oracle (its metrics are then absent).
+    tile_metrics: also the worst per-tile rel-L2 of every input gradient ("tile_grad_in<i>", and the same metric of the
+    comparators), tiles being the backward's tile shape of the input's level (whole samples on a run-time-geometry level).
+    teachers=n: the student's train forward runs in lockstep with n frozen eval-mode teachers (forward_multi, the
+    configuration of DistillStep); "teacher<k>_<level>" is each teacher's output against the fp64 eval oracle (max-rel)."""
     if force_argmax is None:
         force_argmax = True
     from mm_distillnet_b200.bifpn import debug_pool_argmax
     C, cc = 112, [48, 120, 352]
     gen = torch.Generator().manual_seed(seed)
-    cells = [mmd.BiFPN(C, cc, first_time=(i == 0 and first), attention=attention) for i in range(n_cells)]
-    stack = mmd.BiFPNStack(*cells)
-    with torch.no_grad():
-        for k, p in stack.named_parameters():
-            if k[-3:-1] == "_w":
-                if fw_mode == "mixed":
-                    p.copy_(torch.rand(p.shape, generator=gen) * 2.5 - 0.5)
-            elif ".bn." in k or k.endswith(".1.weight") or k.endswith(".1.bias"):
-                if k.endswith("weight"):
-                    p.copy_(torch.rand(p.shape, generator=gen) + 0.5)
-                else:
-                    p.copy_(torch.randn(p.shape, generator=gen) * 0.1)
-        for k, b in stack.named_buffers():
-            if "running_var" in k:
-                b.copy_(torch.rand(b.shape, generator=gen) * 1.5 + 0.5)
-            elif "running_mean" in k:
-                b.copy_(torch.randn(b.shape, generator=gen) * 0.2)
-    params = {k: v.clone() for k, v in stack.state_dict().items()}
-    if first:
-        xs = [torch.randn(B, c, s3 >> i, s3 >> i, generator=gen) for i, c in enumerate(cc)]
-    else:
-        xs = [torch.randn(B, C, max(s3 >> i, 1), max(s3 >> i, 1), generator=gen) for i in range(5)]
-    if dtype != torch.float32:   # compare on identical (rounded) inputs
-        xs = [x.to(dtype).float() for x in xs]
+    H3, W3 = (s3, s3) if isinstance(s3, int) else s3
+
+    def random_stack():
+        cells = [mmd.BiFPN(C, cc, first_time=(i == 0 and first), attention=attention) for i in range(n_cells)]
+        stack = mmd.BiFPNStack(*cells)
+        with torch.no_grad():
+            for k, p in stack.named_parameters():
+                if k[-3:-1] == "_w":
+                    if fw_mode == "mixed":
+                        p.copy_(torch.rand(p.shape, generator=gen) * 2.5 - 0.5)
+                elif ".bn." in k or k.endswith(".1.weight") or k.endswith(".1.bias"):
+                    if k.endswith("weight"):
+                        p.copy_(torch.rand(p.shape, generator=gen) + 0.5)
+                    else:
+                        p.copy_(torch.randn(p.shape, generator=gen) * 0.1)
+            for k, b in stack.named_buffers():
+                if "running_var" in k:
+                    b.copy_(torch.rand(b.shape, generator=gen) * 1.5 + 0.5)
+                elif "running_mean" in k:
+                    b.copy_(torch.randn(b.shape, generator=gen) * 0.2)
+        return stack, {k: v.clone() for k, v in stack.state_dict().items()}
+
+    def random_inputs():
+        if first:
+            xs = [torch.randn(B, c, H3 >> i, W3 >> i, generator=gen) for i, c in enumerate(cc)]
+        else:
+            xs = [torch.randn(B, C, max(H3 >> i, 1), max(W3 >> i, 1), generator=gen) for i in range(5)]
+        if dtype != torch.float32:   # compare on identical (rounded) inputs
+            xs = [x.to(dtype).float() for x in xs]
+        return xs
+
+    stack, params = random_stack()
+    xs = random_inputs()
+    t_stacks, t_params, t_xs = [], [], []
+    for _ in range(teachers):
+        t, tp = random_stack()
+        t_stacks.append(t.to(DEV).eval().requires_grad_(False))   # frozen, as DistillStep's teachers
+        t_params.append(tp)
+        t_xs.append(random_inputs())
     stack = stack.to(DEV)
     m = {}
     # CUDA first: eval forward, then the train forward whose recorded arg-max the oracle follows; its backward runs last
@@ -133,7 +159,21 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
         ev = stack(tuple(to_dev(xs, dtype, channels_last)))
     stack.train()
     xd = [x.requires_grad_(True) for x in to_dev(xs, dtype, channels_last)]
-    tr = stack(tuple(xd))
+    if teachers:
+        from mm_distillnet_b200.bifpn import forward_multi
+        t_xd = [tuple(to_dev(x, dtype, channels_last)) for x in t_xs]
+        outs = forward_multi([(stack, tuple(xd))] + list(zip(t_stacks, t_xd)))
+        tr = outs[0]
+        t_ev = [[o.clone() for o in out] for out in outs[1:]]
+        for k, (tp, x, out) in enumerate(zip(t_params, t_xs, t_ev)):
+            with torch.no_grad():
+                ref = O.bifpn_stack(tuple(v.double() for v in x), {n: (v.double() if v.is_floating_point() else v)
+                                                                   for n, v in tp.items()},
+                                    n_cells, first_cell_first_time=first, training=False, attention=attention)
+            for n, o, r in zip(H.LEVELS, out, ref):
+                m["teacher%d_%s" % (k, n)] = H.max_rel(o.float().cpu(), r)
+    else:
+        tr = stack(tuple(xd))
     hints = debug_pool_argmax(tr[0]) if force_argmax else None
 
     def oracle_run(dt, training):
@@ -155,7 +195,8 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
     tr_ref, xin_ref, leaf_ref = oracle_run(dt_ref, True)
     gouts = [torch.randn(t.shape, generator=gout_seed) for t in tr_ref]
     sum((t * go.to(dt_ref)).sum() for t, go in zip(tr_ref, gouts)).backward()
-    if ref64:
+    ref32 = ref32 and ref64
+    if ref32:
         tr32, xin32, leaf32 = oracle_run(torch.float32, True)
         sum((t * go).sum() for t, go in zip(tr32, gouts)).backward()
     if dtype == torch.bfloat16:   # calibration: the same algorithm executed by PyTorch entirely in bf16
@@ -165,6 +206,9 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
             m["torchbf16_train_" + n] = H.max_rel(trb[i].detach().float(), tr_ref[i].detach())
         for i in range(len(xs)):
             m["torchbf16_grad_in%d" % i] = H.rel_l2(xinb[i].grad.float(), xin_ref[i].grad)
+            if tile_metrics:
+                m["torchbf16_tile_grad_in%d" % i] = H.worst_tile_rel_l2(xinb[i].grad.float(), xin_ref[i].grad,
+                                                                        input_tile(xs[i]))
         fwn = fwd_ = 0.0
         for k, v in leafb.items():   # the all-bf16 run's parameter gradients, worst per class (same metric as ours below)
             if not (torch.is_tensor(v) and v.requires_grad) or k.endswith("conv.bias"):
@@ -186,12 +230,16 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
     sum((t.float() * go.to(DEV)).sum() for t, go in zip(tr, gouts)).backward()
     for i, (n, t, r) in enumerate(zip(H.LEVELS, tr, tr_ref)):
         m["train_" + n] = H.max_rel(t.detach().float().cpu(), r.detach())
-        if ref64:
+        if ref32:
             m["ref32_train_" + n] = H.max_rel(tr32[i].detach(), r.detach())
     for i, x in enumerate(xd):
         m["grad_in%d" % i] = H.rel_l2(x.grad.float().cpu(), xin_ref[i].grad)
-        if ref64:
+        if ref32:
             m["ref32_grad_in%d" % i] = H.rel_l2(xin32[i].grad, xin_ref[i].grad)
+        if tile_metrics:
+            m["tile_grad_in%d" % i] = H.worst_tile_rel_l2(x.grad.float().cpu(), xin_ref[i].grad, input_tile(xs[i]))
+            if ref32:
+                m["ref32_tile_grad_in%d" % i] = H.worst_tile_rel_l2(xin32[i].grad, xin_ref[i].grad, input_tile(xs[i]))
     worst, worst32 = {}, {}
     fw_num = fw_den = fw_num32 = 0.0
     for k, p in stack.named_parameters():
@@ -212,13 +260,13 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
         if cls == "fw":   # all fusion-weight gradients of the stack as ONE vector (see check_fp32)
             fw_num += float((p.grad.cpu().double() - r.double()).pow(2).sum())
             fw_den += float(r.double().pow(2).sum())
-            if ref64:
+            if ref32:
                 fw_num32 += float((leaf32[k].grad.double() - r.double()).pow(2).sum())
         if e > worst.get(cls, 0.0):
             worst[cls] = e
             m["worstname_" + cls] = "%s |g|=%.3e" % (k, r.norm().item())
         worst.setdefault(cls, 0.0)
-        if ref64:
+        if ref32:
             worst32[cls] = max(worst32.get(cls, 0.0), H.rel_l2(leaf32[k].grad, r))
     for k, v in worst.items():
         m["pgrad_" + k] = v
@@ -226,7 +274,7 @@ def random_stack_case(n_cells, first, B, s3, dtype=torch.float32, seed=0, channe
         m["ref32_pgrad_" + k] = v
     if fw_den > 0.0:
         m["pgrad_fwall"] = (fw_num / fw_den) ** 0.5
-        if ref64:
+        if ref32:
             m["ref32_pgrad_fwall"] = (fw_num32 / fw_den) ** 0.5
     return m
 

@@ -98,6 +98,32 @@ def rel_l2(a, b):
     return d / n if n > 0 else d
 
 
+# Tile shapes (TW, TH) of the tiled BiFPN node kernels (bifpn_fwd_v4.cu / bifpn_bwd_v4.cu, pick_geom), tried in this order;
+# a level that fits none of them runs on the run-time-geometry kernels (bifpn_fwd_tc.cu / bifpn_bwd_tc.cu).
+TILE_GEOMS = ((16, 8), (12, 8), (8, 8), (12, 6), (6, 6))
+
+
+def pick_geom(H, W):
+    """Python mirror of pick_geom(): the (TW, TH) tile of an H x W level, or None for the run-time-geometry kernels."""
+    for tw, th in TILE_GEOMS:
+        if W % tw == 0 and H % th == 0:
+            return tw, th
+    return None
+
+
+def worst_tile_rel_l2(a, b, tile):
+    """Largest rel-L2 of a against b over the (TH x TW) tiles of each sample ([B, C, H, W] tensors, all channels of a tile
+    together): one wrong or missing tile reads ~1 here, whatever the size of the rest of the tensor."""
+    tw, th = tile
+    a = torch.as_tensor(a).double()
+    b = torch.as_tensor(b).double()
+    B, C, Hh, W = b.shape
+    assert Hh % th == 0 and W % tw == 0, (tuple(b.shape), tile)
+    per = lambda t: t.reshape(B, C, Hh // th, th, W // tw, tw).pow(2).sum(dim=(1, 3, 5))
+    num, den = per(a - b), per(b)
+    return float((num / den.clamp_min(1e-300)).sqrt().max())
+
+
 def max_rel(a, b):
     """max |a-b| / max|b| : the 'relative' error used for the 1e-4 bar on dense tensors."""
     a = torch.as_tensor(a).double()
