@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define MMD_VERSION 110
+#define MMD_VERSION 111
 
 typedef void* mmd_stream_t; /* cudaStream_t */
 
@@ -255,7 +255,8 @@ enum {
 
 typedef struct {
   int32_t kind;
-  int32_t train;          /* 1: batch statistics, deferred-BN output, running-stat update; 0: running stats folded into the 1x1 conv */
+  int32_t train;          /* 1: batch statistics, deferred-BN output, running-stat update (running stats instead: frozen_bn); */
+                          /* 0: running stats folded into the 1x1 conv                                                         */
   int32_t n_in;
   int32_t swish;          /* NODE: apply x*sigmoid(x) to the fused sum (BiFPN nodes: 1; bare SeparableConvBlock: 0) */
   MmdTensor in[3];
@@ -306,6 +307,13 @@ typedef struct {
   const float* copy_src;  /* COPY */
   float* copy_dst;
   int64_t copy_n;
+  /* frozen BatchNorm (NODE_FWD / PROJ_FWD / NODE_BWD / PROJ_BWD with train = 1): the layer's nn.BatchNorm2d is in eval()   */
+  /* inside a training forward.  mmd_bifpn_prep writes out.bn = (gamma*invstd_r, beta - running_mean*gamma*invstd_r,        */
+  /* running_mean, invstd_r), invstd_r = 1/sqrt(running_var + eps), before the forward; the producer accumulates no         */
+  /* statistics, finalises nothing and leaves running_mean / running_var / num_batches_tracked untouched; the backward     */
+  /* uses A = gamma*invstd_r and no batch-statistics terms (dL/dgamma = sum G*xhat_r, dL/dbeta = sum G as before).         */
+  int32_t frozen_bn;
+  int32_t pad2_;
 } MmdOp;
 
 /* Packed parameter block of one NODE / PROJ op (bf16 storage only; every section starts 128-byte aligned):
@@ -321,7 +329,9 @@ size_t mmd_packed_bytes(int32_t kind, int32_t Cin, int32_t C);
  * current fp32 parameters (and, in eval mode, the running statistics).  One or two launches for a whole stack.  Call it
  * whenever the parameters may have changed since the last call (every training step; once for frozen teachers).
  * COPY ops of the list run first, for both dtypes.  An op with train = 0 that saves its depthwise output (save_d) is a
- * header that will be differentiated: its backward operand is packed as well. */
+ * header that will be differentiated: its backward operand is packed as well.  The BatchNorm vector (out.bn) of every op
+ * with frozen_bn = 1 is written here too, for both dtypes (bf16: by the packing launch, fp32: one launch of its own), so
+ * a training forward with frozen layers must call this before mmd_bifpn_run / _run_multi with the same bases. */
 int mmd_bifpn_prep(const MmdOp* ops, int32_t n_ops, void* const* bases, int32_t n_bases, int32_t C, int32_t dtype,
                    mmd_stream_t stream);
 

@@ -95,6 +95,7 @@ class Op(C.Structure):
         ("aux", Ref), ("praw", Ref),
         ("head_K", C.c_int32), ("head_tot", C.c_int32), ("head_off", C.c_int32), ("head_act", C.c_int32),
         ("copy_src", C.c_void_p), ("copy_dst", C.c_void_p), ("copy_n", C.c_int64),
+        ("frozen_bn", C.c_int32), ("pad2_", C.c_int32),
     ]
 
 

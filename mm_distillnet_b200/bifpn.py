@@ -212,7 +212,7 @@ class _Tn:
 class _OpN:
     __slots__ = ("kind", "ins", "modes", "conv", "bn", "dw", "fw", "fw_eps", "swish", "out", "save_d", "pidx",
                  "stats", "counter", "du", "slots", "glike", "bwd_counter", "cin", "gref", "packed", "aux", "praw", "tag",
-                 "train", "gover", "head", "copy", "gpad", "dxref")
+                 "train", "gover", "head", "copy", "gpad", "dxref", "frozen")
 
     def __init__(self, kind):
         self.kind = kind
@@ -238,6 +238,7 @@ class _OpN:
         self.copy = None       # COPY: (source tensor, destination pointer, floats)
         self.gpad = []         # HEAD_GATHER: (base, off) of the padded gradient of each input
         self.dxref = None      # ACT_FWD: (base, off) of the gradient its backward writes
+        self.frozen = False    # NODE / PROJ of a training plan whose BatchNorm is in eval(): running statistics, no update
 
 
 # fixed base indices
@@ -284,10 +285,12 @@ def _ptr(t):
 
 
 class _Plan:
-    """Op lists + arena layout for one (cells, shapes, dtype, mode) combination."""
+    """Op lists + arena layout for one (cells, shapes, dtype, mode) combination.  `frozen`: ids of the nn.BatchNorm2d
+    modules that a training plan normalises with their running statistics (layers in eval() inside a train() module)."""
 
-    def __init__(self, mods, kind, in_shapes, dtype, train, need_grad, in_need_grad):
+    def __init__(self, mods, kind, in_shapes, dtype, train, need_grad, in_need_grad, frozen=()):
         self.train, self.need_grad = train, need_grad and train
+        self.frozen = frozenset(frozen) if train else frozenset()
         self.dtype = dtype
         self.esize = 4 if dtype == torch.float32 else 2
         self.B = in_shapes[0][0]
@@ -371,6 +374,7 @@ class _Plan:
         op.ins = [t for t, _ in ins]
         op.modes = [m for _, m in ins]
         op.conv, op.bn, op.dw = sep.pointwise_conv.conv, sep.bn, sep.depthwise_conv.conv
+        op.frozen = train is not False and id(sep.bn) in self.frozen
         op.fw, op.fw_eps, op.swish = fw, fw_eps, swish
         H = ins[0][0].H if ins[0][1] == _lib.IN_SAME else None
         W = ins[0][0].W if ins[0][1] == _lib.IN_SAME else None
@@ -409,6 +413,7 @@ class _Plan:
         op = _OpN(_lib.OP_PROJ_FWD)
         op.ins, op.modes = [x], [_lib.IN_SAME]
         op.conv, op.bn = seq[0].conv, seq[1]
+        op.frozen = id(seq[1]) in self.frozen
         op.cin = x.C
         op.out = self._new_raw(x.H, x.W, seq[1])
         op.out.producer = op
@@ -597,6 +602,7 @@ class _Plan:
         o.out = _tensor(op.out)
         o.save_d = _ref(op.save_d)
         o.packed = _ref(op.packed)
+        o.frozen_bn = 1 if op.frozen else 0
         for i in range(3):
             o.pidx[i] = _ref(op.pidx[i])
             o.in_slot[i] = _ref(op.slots[i])
@@ -981,8 +987,9 @@ class _Runner:
                 raise ValueError("BiFPN: inputs must be [B,C,H,W] tensors sharing batch, dtype and device")
         ck = tuple(id(m) for m in mods)
         if self._param_cache is None or self._param_cache[0] != ck:   # walking 5 cells' modules costs ~1 ms per call
-            self._param_cache = (ck, [p for m in mods for p in m.parameters()], [b for m in mods for b in m.buffers()])
-        params, buffers = self._param_cache[1], self._param_cache[2]
+            self._param_cache = (ck, [p for m in mods for p in m.parameters()], [b for m in mods for b in m.buffers()],
+                                 [b for m in mods for b in m.modules() if isinstance(b, nn.BatchNorm2d)])
+        params, buffers, bns = self._param_cache[1], self._param_cache[2], self._param_cache[3]
         if len(params) == 0:
             raise RuntimeError("mm_distillnet_b200.BiFPN: the module holds no parameters (an nn.DataParallel replica?); "
                                "multi-GPU runs use one process per GPU, see mm_distillnet_b200.DistillStep")
@@ -1010,11 +1017,16 @@ class _Runner:
         # the op lists hold the raw data_ptr() of EVERY parameter and BatchNorm buffer: all of them are part of the key
         # (load_state_dict(assign=True), an EMA swap through p.data or a reassigned buffer must miss the cache)
         ptrs = hash(tuple(t.data_ptr() for t in params) + tuple(t.data_ptr() for t in buffers))
+        # training plans follow each BatchNorm layer's own mode: a layer in eval() (frozen BatchNorm) normalises with its
+        # running statistics and leaves them alone.  The per-layer mask is part of the key, so a mode change between two
+        # calls builds or reuses the matching plan (eval plans fold every BatchNorm whatever its flag says)
+        mask = tuple(m.training for m in bns) if training else ()
         key = (kind, tuple(tuple(x.shape) for x in inputs), x0.dtype, bool(training), need_grad, tuple(in_need),
-               x0.device.index, len(params), ptrs)
+               x0.device.index, len(params), ptrs, mask)
         plan = self.plans.get(key)
         if plan is None:
-            plan = _Plan(mods, kind, [tuple(x.shape) for x in inputs], x0.dtype, bool(training), need_grad, in_need)
+            frozen = [id(m) for m, on in zip(bns, mask) if not on]
+            plan = _Plan(mods, kind, [tuple(x.shape) for x in inputs], x0.dtype, bool(training), need_grad, in_need, frozen)
             plan.device = x0.device
             self.plans[key] = plan
             if len(self.plans) > 16:
@@ -1055,8 +1067,9 @@ class _Runner:
     def _prep(self, plan, bases):
         """(Re)build the packed parameter blocks when the parameters may have changed: every training forward (the
         optimiser updates the weights between steps); for eval plans (frozen teachers) only when a parameter / buffer
-        version or the global running-statistics epoch moved."""
-        if plan.dtype != torch.bfloat16 and not plan.copies:
+        version or the global running-statistics epoch moved.  Training plans with frozen BatchNorm layers also get
+        those layers' (scale, shift, mean, invstd) vectors rewritten here, in fp32 too: gamma and beta move every step."""
+        if plan.dtype != torch.bfloat16 and not plan.copies and not plan.frozen:
             return
         if plan.train:
             for m in plan.mods:   # this forward updates running statistics through raw pointers

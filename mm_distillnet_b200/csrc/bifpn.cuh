@@ -123,7 +123,24 @@ struct NodeFwdP {
   // statistics and clears the accumulators.
   BnSrc bnsrc[3];
   int defer_bn;
+  // Frozen BatchNorm (MmdOp::frozen_bn): out_bn already holds the running-statistics vector (frozen_bn_vector, written by
+  // mmd_bifpn_prep); the producer accumulates no statistics, finalises nothing and never touches the running statistics.
+  int frozen_bn;
 };
+
+// out_bn of a frozen BatchNorm (the layer is in eval() inside a training forward): PyTorch's eval-mode normalisation
+// y = gamma * (x - running_mean) / sqrt(running_var + eps) + beta as the (scale, shift, mean, invstd) vector the consumers
+// apply on load and the backward reads.
+template <int C>
+__device__ __forceinline__ void frozen_bn_vector(int c, const float* gamma, const float* beta, const float* rm, const float* rv,
+                                                 float eps, float* out_bn) {
+  const float invstd = (float)(1.0 / sqrt((double)rv[c] + (double)eps));
+  const float scale = gamma[c] * invstd;
+  out_bn[c] = scale;
+  out_bn[C + c] = beta[c] - rm[c] * scale;
+  out_bn[2 * C + c] = rm[c];
+  out_bn[3 * C + c] = invstd;
+}
 
 // (scale, shift) of channel c of input `t`: from the finalised vector, or rebuilt from the producer's statistics
 template <int C>
@@ -218,6 +235,7 @@ struct NodeBwdP {
   unsigned* counter;
   TileGeom g;
   int defer_fw;   // 1: node_bwd_b4 leaves the fusion-weight gradient to fwgrad_kernel (one launch per backward)
+  int frozen_bn;  // 1: the BatchNorm of `out` normalised with its running statistics (see bn_bwd_coefs)
 };
 
 // Deferred fusion-weight gradients: the slots (sum du, sum du * xhat per input edge) of every node are complete when the

@@ -63,6 +63,8 @@ __device__ __forceinline__ void cons_weights(const NodeBwdP& P, float (&cw)[3]) 
 }
 
 // BN backward coefficients per channel: dL/dx_raw = A*G + Bc*x_raw + Cc  (SURVEY.md A.3), from the consumers' slots.
+// A frozen BatchNorm (eval-mode layer in a training forward) normalised with constants: A = gamma*invstd_r, Bc = Cc = 0;
+// the slots still give dL/dbeta = S1 and dL/dgamma = S2 (their xhat is taken against the running statistics of out_bn).
 template <int C>
 __device__ __forceinline__ void bn_bwd_coefs(const NodeBwdP& P, const float (&cw)[3], float* s_coef) {
   const int tid = threadIdx.x;
@@ -75,8 +77,8 @@ __device__ __forceinline__ void bn_bwd_coefs(const NodeBwdP& P, const float (&cw
     const double n = (double)P.g.B * P.g.H * P.g.W;
     const float gamma = P.bn_w[tid], mean = P.out_bn[2 * C + tid], invstd = P.out_bn[3 * C + tid];
     const float A = gamma * invstd;
-    const float Bc = (float)(-(double)gamma * invstd * invstd * S2 / n);
-    const float Cc = (float)(-(double)A * S1 / n - (double)Bc * mean);
+    const float Bc = P.frozen_bn ? 0.f : (float)(-(double)gamma * invstd * invstd * S2 / n);
+    const float Cc = P.frozen_bn ? 0.f : (float)(-(double)A * S1 / n - (double)Bc * mean);
     s_coef[tid] = A;
     s_coef[C + tid] = Bc;
     s_coef[2 * C + tid] = Cc;

@@ -70,6 +70,7 @@ __device__ __forceinline__ void tile_epilogue(float (&acc)[8][C / 16], const flo
 // ---- BatchNorm finalisation by the last CTA -----------------------------------------------------------------
 template <int C>
 __device__ __forceinline__ void bn_finalize(const NodeFwdP& P, double st_sum, double st_sq, int* s_flag) {
+  if (P.frozen_bn) return;   // running-statistics vector written by mmd_bifpn_prep; nothing to accumulate or update
   const int tid = threadIdx.x;
   if (tid < C) {
     atomicAdd(P.stats + tid, st_sum);

@@ -89,6 +89,7 @@ __device__ __forceinline__ void tile_epilogue_tc(uint32_t tmem_base, const float
 
 template <int C>
 __device__ __forceinline__ void bn_finalize_tc(const NodeFwdP& P, double st_sum, double st_sq, int* s_flag) {
+  if (P.frozen_bn) return;   // running-statistics vector written by mmd_bifpn_prep; nothing to accumulate or update
   const int tid = threadIdx.x;
   const TileGeom& g = P.g;
   if (tid < C) {

@@ -573,10 +573,10 @@ __device__ __forceinline__ void node_fwd_body(const NodeFwdP& P, const NodeFwdP&
   if (!pack_ready) tc::mbar_wait(bar_pack, X.ph_pack);   // a CTA without tiles still consumes this node's pack phase
   X.ph_pack ^= 1u;
 
-  // ---- BatchNorm statistics (+ finalisation by the last CTA of this network unless it is deferred)
+  // ---- BatchNorm statistics (+ finalisation by the last CTA of this network unless it is deferred; none when frozen)
   tc::fence_before_sync();
   __syncthreads();
-  if (!train) return;
+  if (!train || P.frozen_bn) return;
   double* s_red = reinterpret_cast<double*>(r1);   // [4 slices][C/2 pairs][4]
   if (ss < 4) {
 #pragma unroll

@@ -42,11 +42,14 @@ static int fill_fwd(const MmdOp& op, const Bases& B, int batch, NodeFwdP& p) {
   p.bn_mom = op.bn_momentum;
   p.g = make_geom(batch, op.out.H, op.out.W);
   p.defer_bn = 0;
+  p.frozen_bn = 0;
   for (int i = 0; i < 3; ++i) p.bnsrc[i] = BnSrc{nullptr, nullptr, nullptr, 0.0, 0.f};
   MMD_CHECK_ARG(p.out != nullptr, "op: no output");
   if (op.kind != MMD_OP_BNAPPLY && op.kind != MMD_OP_POOLFUSE) {
     MMD_CHECK_ARG(p.pw_w && p.pw_b && p.bn_w && p.bn_b && p.bn_rm && p.bn_rv, "op: missing conv/bn parameters");
     if (op.train) MMD_CHECK_ARG(p.out_bn && p.stats && p.counter, "train op: missing bn/stats/counter storage");
+    MMD_CHECK_ARG(!op.frozen_bn || (op.train && p.out_bn), "op: a frozen BatchNorm needs train = 1 and a BatchNorm vector");
+    p.frozen_bn = op.frozen_bn ? 1 : 0;
   }
   return 0;
 }
@@ -99,6 +102,7 @@ static int fill_bwd(const MmdOp& op, const Bases& B, int batch, NodeBwdP& p) {
   p.counter = B.get<unsigned>(op.counter);
   p.g = make_geom(batch, op.out.H, op.out.W);
   p.defer_fw = 0;
+  p.frozen_bn = (op.kind == MMD_OP_NODE_BWD || op.kind == MMD_OP_PROJ_BWD) && op.frozen_bn ? 1 : 0;
   return 0;
 }
 
@@ -113,7 +117,8 @@ struct DeferPlan {
 static bool ref_eq(const MmdRef& a, const MmdRef& b) { return a.base >= 0 && a.base == b.base && a.off == b.off; }
 
 // A train-mode NODE_FWD / PROJ_FWD op may defer when every later op that applies its BatchNorm on load runs on a kernel
-// that can rebuild the coefficients from the statistics: the v4 node kernel, the poolfuse pre-pass, bnapply.
+// that can rebuild the coefficients from the statistics: the v4 node kernel, the poolfuse pre-pass, bnapply.  A frozen
+// BatchNorm has no statistics: its vector is written before the forward and its consumers read it as it is.
 static int plan_defer(const MmdOp* ops, int n_ops, const Bases& B, int batch, int dtype, DeferPlan& D) {
   D.defer.assign(n_ops, 0);
   D.src.assign((size_t)n_ops * 3, BnSrc{nullptr, nullptr, nullptr, 0.0, 0.f});
@@ -121,7 +126,7 @@ static int plan_defer(const MmdOp* ops, int n_ops, const Bases& B, int batch, in
   if (dtype != MMD_BF16 || tc_disabled() || !bn_deferral_enabled()) return 0;
   for (int j = 0; j < n_ops; ++j) {
     const MmdOp& op = ops[j];
-    if (!op.train || !(op.kind == MMD_OP_NODE_FWD || (op.kind == MMD_OP_PROJ_FWD && op.Cin % 8 == 0))) continue;
+    if (!op.train || op.frozen_bn || !(op.kind == MMD_OP_NODE_FWD || (op.kind == MMD_OP_PROJ_FWD && op.Cin % 8 == 0))) continue;
     if (op.out.bn.base < 0 || op.stats.base < 0) continue;
     bool ok = true;
     for (int k = j + 1; k < n_ops && ok; ++k) {

@@ -7,6 +7,10 @@
 //   bias              : fp32 [C] (eval: folded)
 //   taps              : fp32 [9][C] (depthwise [C,1,3,3] transposed to tap-major)
 //   backward B operand: bf16 [C/8][C][8], element (o, i) of W stored at [o/8][i][o%8]  (dL/dd = dy * W)
+//
+// It also writes the BatchNorm vector of every frozen layer (MmdOp::frozen_bn) from gamma, beta and the running
+// statistics: every training forward, since gamma and beta move every step.  bf16 plans do it in the packing launch,
+// fp32 plans (no packed blocks) in one frozen_bn_kernel launch.
 #include "bifpn.cuh"
 
 namespace mmd {
@@ -14,6 +18,7 @@ namespace mmd {
 struct PrepDesc {
   const float *pw_w, *pw_b, *bn_w, *bn_b, *bn_rm, *bn_rv, *dw_w;
   unsigned char* dst;
+  float* frozen_bn;   // non-null: out.bn of a frozen BatchNorm, written from bn_w / bn_b / bn_rm / bn_rv
   int Cin, Kp, train, node, NC, nchunks, bwd;
   int offBias, offTaps, offBwd;
   float eps;
@@ -60,6 +65,7 @@ __global__ void __launch_bounds__(256) prep_kernel(const __grid_constant__ PrepA
       bia = (bia - D.bn_rm[c]) * sc + D.bn_b[c];
     }
     reinterpret_cast<float*>(D.dst + D.offBias)[c] = bia;
+    if (D.frozen_bn) frozen_bn_vector<C>(c, D.bn_w, D.bn_b, D.bn_rm, D.bn_rv, D.eps, D.frozen_bn);
   }
   if (!D.node) {
     if (!D.bwd) return;
@@ -96,6 +102,24 @@ __global__ void __launch_bounds__(256) prep_kernel(const __grid_constant__ PrepA
   }
 }
 
+// fp32 plans: the frozen BatchNorm vectors on their own, one CTA per layer
+struct FrozenBnDesc {
+  const float *gamma, *beta, *rm, *rv;
+  float* out_bn;
+  float eps;
+};
+constexpr int kFrozenMax = 64;
+struct FrozenBnArgs {
+  FrozenBnDesc d[kFrozenMax];
+};
+static_assert(sizeof(FrozenBnArgs) <= 4096 && sizeof(PrepArgs) <= 4096, "kernel parameter space");
+
+template <int C>
+__global__ void __launch_bounds__(128) frozen_bn_kernel(const __grid_constant__ FrozenBnArgs A) {
+  const FrozenBnDesc& D = A.d[blockIdx.x];
+  if (threadIdx.x < C) frozen_bn_vector<C>(threadIdx.x, D.gamma, D.beta, D.rm, D.rv, D.eps, D.out_bn);
+}
+
 }  // namespace mmd
 
 using namespace mmd;
@@ -115,8 +139,25 @@ extern "C" int mmd_bifpn_prep(const MmdOp* ops, int32_t n_ops, void* const* base
       const int rc = launch_copy_f32(ops[i].copy_src, ops[i].copy_dst, (long long)ops[i].copy_n, stream);
       if (rc) return rc;
     }
-  if (dtype != MMD_BF16) return 0;   // the fp32 parity kernels read the fp32 parameters directly
   Bases B{bases, n_bases};
+  // frozen BatchNorm vectors that no packing launch writes (fp32 plans, ops without a packed block)
+  FrozenBnArgs fargs;
+  int nf = 0;
+  for (int i = 0; i < n_ops; ++i) {
+    const MmdOp& op = ops[i];
+    if (!op.frozen_bn || (op.kind != MMD_OP_NODE_FWD && op.kind != MMD_OP_PROJ_FWD)) continue;
+    MMD_CHECK_ARG(op.train && op.bn_w && op.bn_b && op.bn_rm && op.bn_rv && B.get<float>(op.out.bn) != nullptr,
+                  "prep: frozen op %d misses its BatchNorm parameters or vector", i);
+    if (dtype == MMD_BF16 && B.get<unsigned char>(op.packed) != nullptr) continue;   // prep_kernel writes it
+    MMD_CHECK_ARG(nf < kFrozenMax, "prep: more than %d frozen BatchNorm layers in one op list", kFrozenMax);
+    fargs.d[nf++] = FrozenBnDesc{op.bn_w, op.bn_b, op.bn_rm, op.bn_rv, B.get<float>(op.out.bn), op.bn_eps};
+  }
+  if (nf > 0) {
+    frozen_bn_kernel<112><<<nf, 128, 0, stream>>>(fargs);
+    MMD_LAUNCH_CHECK();
+    pdl_fence_next();
+  }
+  if (dtype != MMD_BF16) return 0;   // the fp32 parity kernels read the fp32 parameters directly
   PrepArgs args;
   int n = 0;
   auto flush = [&]() -> int {
@@ -141,6 +182,7 @@ extern "C" int mmd_bifpn_prep(const MmdOp* ops, int32_t n_ops, void* const* base
     D.pw_w = op.pw_w; D.pw_b = op.pw_b; D.bn_w = op.bn_w; D.bn_b = op.bn_b;
     D.bn_rm = op.bn_rm; D.bn_rv = op.bn_rv; D.dw_w = op.dw_w;
     D.dst = dst;
+    D.frozen_bn = op.frozen_bn ? B.get<float>(op.out.bn) : nullptr;
     D.Cin = Cin; D.Kp = L.Kp; D.train = op.train; D.node = node ? 1 : 0;
     D.bwd = (op.train || op.save_d.base >= 0) ? 1 : 0;
     D.offBias = L.offBias; D.offTaps = L.offTaps; D.offBwd = L.offBwd;

@@ -178,6 +178,10 @@ class DistillStep:
         few microseconds each: replaying it as one graph takes the host (and any driver contention, e.g. a clock
         monitor) out of the critical path.  Returns self; use replay().
 
+        The graph keeps the BatchNorm modes of the student's layers as they were at capture time (frozen BatchNorm:
+        layers in eval() inside the train-mode student); after switching a layer between train() and eval(), call
+        capture() again — replays do not check the modes.
+
         `double_buffer=True` captures the step TWICE over two static input sets: prefetch() fills the set the running
         graph does not read and replay_prefetched() replays that set's graph, so the pipelined feed needs no
         staging-to-static copy (2 x 236 MB of HBM traffic per step at B = 32).  Both graphs leave the averaged gradient

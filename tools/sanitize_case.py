@@ -86,3 +86,21 @@ for _ in range(3):
     opt.step(flat)
 torch.cuda.synchronize()
 print("adam ok", int(opt.step_count), float(ps[1].abs().mean()))
+
+# frozen BatchNorm: every other node's BatchNorm in eval() inside a training stack (frozen vector written by the prep
+# launch, no statistics, constant-coefficient BatchNorm backward), plus a frozen head level
+for dtype in (torch.bfloat16, torch.float32):
+    stack = mmd.BiFPNStack(*[mmd.BiFPN(112, CC, first_time=(i == 0)) for i in range(2)]).to(dev).train()
+    bns = [m for m in stack.modules() if isinstance(m, torch.nn.BatchNorm2d)]
+    for m in bns[::2]:
+        m.eval()
+    xs = [torch.randn(1, c, 48 >> i, 48 >> i, device=dev).to(dtype).contiguous(memory_format=torch.channels_last).requires_grad_(True)
+          for i, c in enumerate(CC)]
+    out = stack(tuple(xs))
+    reg = mmd.Regressor(112, 9, 3).to(dev).train()
+    for m in reg.bn_list[2]:
+        m.eval()
+    r, ar = reg(out)
+    (sum(o.float().mean() for o in out) + r.float().mean() + ar.float().mean()).backward()
+    torch.cuda.synchronize()
+    print(dtype, "frozen BatchNorm ok", int(bns[0].num_batches_tracked), int(bns[1].num_batches_tracked))
